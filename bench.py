@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4|c5]   # this repo's sm_100a path
     python bench.py --impl reference --gpus N ...                          # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's results as DIR/<name>.npy
 
 Workloads (BASELINE.json configs; ``--config``, default c2 = the configuration the metric is quoted on):
   c2  predict_memory full CWE memory, bert-base, seq_len 512, 64 issue reports / GPU, 129 anchors
@@ -42,6 +43,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (which may be read-only)
 
 SEQ, SEED = 512, 2021
 METRIC, UNIT = "issue-reports/sec, bert-base seq512 + CWE memory", "issues/s"
@@ -273,11 +275,40 @@ def cpu_oracle_throughput(ids, mask, tids, bank, same_idx, budget_s: float = 14.
     return rec, ref, n
 
 
+DUMP_BYTES = 64_000_000            # --dump-outputs: all files together stay within 64 MB
+
+
+def write_outputs(out_dir, arrays):
+    """``--dump-outputs``: one ``out_dir/<name>.npy`` per result array, float32 (integer arrays as float64, which holds
+    them exactly), so that two builds can be compared output for output on the same seeded inputs.  When the
+    [B, G, 2] arrays (logits, probs) would take the total over DUMP_BYTES (config c4), they keep a seeded random subset
+    of the anchors, the same one in every run with the same arguments, listed in ``anchor_index.npy``."""
+    import numpy as np
+    import torch
+    out = {k: v.numpy().astype(np.float32 if v.is_floating_point() else np.float64) for k, v in arrays.items()}
+    wide = [k for k, a in out.items() if a.ndim == 3]
+    budget = DUMP_BYTES - 256 * (len(out) + 1)                        # .npy headers
+    total = sum(a.nbytes for a in out.values())
+    if wide and total > budget:
+        G = out[wide[0]].shape[1]
+        per_anchor = sum(out[k][:, :1].nbytes for k in wide) + 8      # + its entry in anchor_index
+        keep = max(1, (budget - (total - G * (per_anchor - 8))) // per_anchor)
+        idx = torch.randperm(G, generator=torch.Generator().manual_seed(SEED))[:keep].sort().values.numpy()
+        out = {k: (a[:, idx] if k in wide else a) for k, a in out.items()}
+        out["anchor_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
+    written = sum(os.path.getsize(os.path.join(out_dir, k + ".npy")) for k in out)
+    if written > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs wrote {written} bytes, more than {DUMP_BYTES}")
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warm = max(args.steps or 20, 1), max(args.warmup, 0)
+    steps, warm = args.steps or 20, max(args.warmup, 0)
     import torch
     from oracle import memvul_oracle as O
     cfg = CONFIGS[args.config]
@@ -293,22 +324,20 @@ def run_reference(args):
         for _ in range(min(warm, 2)):
             O.memory_forward(sd, ids, mask, tids, bank, 0)
         t0 = time.perf_counter()
-        done = 0
         for _ in range(steps):
-            O.memory_forward(sd, ids, mask, tids, bank, 0)
-            done += 1
-            if time.perf_counter() - t0 > 150:
-                break
+            last = O.memory_forward(sd, ids, mask, tids, bank, 0)
         dt = time.perf_counter() - t0
-    v = done * b / dt
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, last)
+    v = steps * b / dt
     single = single_thread_figure(O, sd, ids, mask, tids, bank, 0, cores)
-    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": done,
-            "warmup": min(warm, 2), "ms_per_step": dt / done * 1e3, "higher_is_better": True, "scaling": "weak",
+    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
+            "warmup": min(warm, 2), "ms_per_step": dt / steps * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"{cfg['name']}; CPU sample of {b} issue reports per step (G={G})",
                        "note": "reference = CPU fp32 PyTorch restatement of ModelMemory.forward (oracle port); AllenNLP is not installable offline"},
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
-                             "sample": f"{done} steps x {b} issue reports, S<={SEQ}, {torch.get_num_threads()} threads",
+                             "sample": f"{steps} steps x {b} issue reports, S<={SEQ}, {torch.get_num_threads()} threads",
                              "single_thread": single, "host": host_cpu()},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line), flush=True)
@@ -426,7 +455,7 @@ def run_native(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, t0, t1
+        return ms, t0, t1, last
 
     with torch.no_grad():
         for _ in range(warm):
@@ -435,7 +464,7 @@ def run_native(args):
             gather.wait()
         torch.cuda.synchronize()
         # ---- calibrate: step time -> number of pre-heat steps and (when --steps is not given) of timed steps
-        ms_cal, _, _ = timed(step_resident, 3)
+        ms_cal = timed(step_resident, 3)[0]
         step_ms = ms_cal / 3
         steps = args.steps if args.steps else max(20, int(3200.0 / step_ms) + 1)      # default: >= 3 s timed region
         preheat_steps = int(args.preheat_s * 1e3 / step_ms) if args.preheat_s > 0 else 0
@@ -452,9 +481,12 @@ def run_native(args):
             sampler.start()
             time.sleep(0.06)
         l0 = native.launch_count()
-        ms_res, t0, t1 = timed(step_resident, steps)
+        ms_res, t0, t1, res_timed = timed(step_resident, steps)
         launches = native.launch_count() - l0
         clocks = sampler.stop(t0, t1) if rank == 0 else None
+        # what a caller of match_batch received from the last timed step (rank 0's shard when N > 1)
+        dumped = {k: v.cpu() for k, v in res_timed.items() if not k.startswith("_")} \
+            if args.dump_outputs and rank == 0 else None
 
         for _ in range(2):
             step_e2e()["probs"].numpy()
@@ -462,7 +494,7 @@ def run_native(args):
         def drain(last):                      # the step's result is read on the host inside the timed region
             last["probs"].numpy()
             model.get_metrics(reset=False)
-        ms_e2e, _, _ = timed(step_e2e, steps, after=drain)
+        ms_e2e = timed(step_e2e, steps, after=drain)[0]
         model.get_metrics(reset=True)
 
         # live per-kernel timing: same step with CUDA events around every launch, right after ~1 s of un-instrumented
@@ -569,6 +601,8 @@ def run_native(args):
         del model
         torch.cuda.empty_cache()
         line["anchor_match"] = anchor_match_bench(dev, peaks)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -577,14 +611,18 @@ def run_native(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=0, help="timed steps (default: enough for a >= 3 s timed region)")
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: enough for a >= 3 s timed region)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--preheat-s", type=float, default=3.0, help="untimed pre-heat before the timed steps (sustained clocks)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-anchor-bench", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (<= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus > 1 and world == 1 and args.impl == "native":
         # convenience: re-launch under torchrun when called directly with --gpus N

@@ -1,11 +1,11 @@
 """On-hardware precision evidence (VERDICT r01 item 10): the GPU path (fp16 operands, fp32 accumulate / residual stream)
-against the CPU oracle over 1,024 S=512 issue reports x 129 anchors, with the match head (``_projector``) scaled x1, x4
+against the CPU oracle over 768 S=512 issue reports x 129 anchors, with the match head (``_projector``) scaled x1, x4
 and x16 -- the logit error grows with the head scale, the 1e-3 gate of BASELINE.json's north_star does not.
 
     python tools/precision_gpu.py [--out profiles/r02_precision.json]
 
-The oracle's header outputs come from tests/golden/precision_u1024.npz (oracle/make_precision_fixture.py, generated in
-the build container); the match itself is re-evaluated here in float64 for every scale from (u, bank)."""
+The oracle's header outputs come from tests/golden/precision_u768.npz (made on the CPU by oracle/make_precision_fixture.py);
+the match itself is re-evaluated here in float64 for every scale from (u, bank)."""
 import argparse
 import json
 import os
@@ -38,7 +38,7 @@ def main():
                     help="split_fp16 = the opt-in accuracy mode (MEMVUL_ENC_PRECISE)")
     ap.add_argument("--rows", type=int, default=0, help="use only the first N rows of the fixture (the accuracy mode is slow)")
     args = ap.parse_args()
-    z = np.load(os.path.join(ROOT, "tests", "golden", "precision_u1024.npz"))
+    z = np.load(os.path.join(ROOT, "tests", "golden", "precision_u768.npz"))
     u_ref, bank_ref = torch.from_numpy(z["u"]), torch.from_numpy(z["bank"])
     seed, n_rows = int(z["seed"]), int(z["rows"])
     if args.rows:
