@@ -4,12 +4,16 @@
 // A LayerNorm row needs all 768 outputs, but one CTA pair's TMEM holds only a 256-column accumulator (twice).  So a
 // CLUSTER OF SIX CTAs = three cta_group::2 pairs works on one 256-row block: pair p owns columns [256p, 256p+256),
 // each CTA 128 of the rows.  Per tile, in every CTA's epilogue warps:
-//   pass 1  v = acc + bias + resid (residual 32x32 boxes arrive by TMA, 2 in flight); row sums of v and v^2;
-//           v is written BACK INTO TMEM (tcgen05.st) -- the accumulator stage doubles as the stash for pass 2;
-//   exchange each thread publishes its (sum, sumsq) for (row, column half) into the shared memory of the three CTAs
+//   pass 1  v = acc + bias + resid (residual 32x32 boxes arrive by TMA, 2 in flight); per-thread statistics of its
+//           128 values, accumulated SHIFTED by a pivot piv (the mean of its first 32 values): the sums of d = v - piv
+//           and d^2 give the partial's mean and centred sum of squares M2 -- never sum(v^2) - n mean^2, which cancels
+//           catastrophically when |mean| >> spread; v is written BACK INTO TMEM (tcgen05.st) -- the accumulator stage
+//           doubles as the stash for pass 2;
+//   exchange each thread publishes its (mean, M2) for (row, column half) into the shared memory of the three CTAs
 //           that own the same rows (st.shared::cluster), then a release/acquire mbarrier round at cluster scope;
-//   pass 2  mean / rstd from the 6 partials; y = (v - mean) * rstd * gamma + beta is staged in swizzled smem and
-//           leaves by TMA store twice: fp32 (the residual stream) and fp16 (the next GEMM's A operand).
+//   pass 2  mean / rstd from the 6 partials by the parallel-variance (Chan et al.) combination, M2 = sum M2_p +
+//           128 sum (mean_p - mean)^2; y = (v - mean) * rstd * gamma + beta is staged in swizzled smem and leaves by TMA
+//           store twice: fp32 (the residual stream) and fp16 (the next GEMM's A operand).
 // This removes the stand-alone LayerNorm kernels (9-13 % of the step in r01c/r01d) and the fp32 round trip of the
 // pre-LN sum through HBM: 10 bytes per element instead of 18.
 // Main loop, barriers and roles are those of gemm_tcgen05_2cta.cuh (warp 0 TMA, warp 1 MMA issue on even ranks,
@@ -278,7 +282,8 @@ gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
       const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
                               static_cast<uint32_t>(acc * Cfg::BN + half_sel * 128);
       // ---------------- pass 1: v = acc + bias + resid -> TMEM, row statistics ----------------
-      float s1 = 0.f, s2 = 0.f;
+      // shifted sums: d = v - piv with piv near the partial's mean, so s1 / s2 stay O(128 spread^2) whatever the row mean
+      float s1 = 0.f, s2 = 0.f, piv = 0.f;
       uint32_t r[2][32];
       tmem_ld_32x32b_x32(t_addr, r[0]);
 #pragma unroll
@@ -302,10 +307,21 @@ gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
           const float v1 = __uint_as_float(a[4 * u + 1]) + bb.y + x.y;
           const float v2 = __uint_as_float(a[4 * u + 2]) + bb.z + x.z;
           const float v3 = __uint_as_float(a[4 * u + 3]) + bb.w + x.w;
-          s1 += (v0 + v1) + (v2 + v3);
-          s2 = fmaf(v0, v0, fmaf(v1, v1, fmaf(v2, v2, fmaf(v3, v3, s2))));
           v[4 * u + 0] = __float_as_uint(v0); v[4 * u + 1] = __float_as_uint(v1);
           v[4 * u + 2] = __float_as_uint(v2); v[4 * u + 3] = __float_as_uint(v3);
+        }
+        if (c == 0) {                                      // pivot = mean of the first 32 values: within O(spread / 6) of
+          float q4[4] = {0.f, 0.f, 0.f, 0.f};              // the partial's mean, so s2 - s1^2 / 128 barely cancels
+#pragma unroll
+          for (int i = 0; i < 32; ++i) q4[i & 3] += __uint_as_float(v[i]);
+          piv = ((q4[0] + q4[1]) + (q4[2] + q4[3])) * (1.0f / 32.0f);
+        }
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {                      // separate sweep: folded into the loop above, ptxas spills
+          const float d0 = __uint_as_float(v[4 * u + 0]) - piv, d1 = __uint_as_float(v[4 * u + 1]) - piv;
+          const float d2 = __uint_as_float(v[4 * u + 2]) - piv, d3 = __uint_as_float(v[4 * u + 3]) - piv;
+          s1 += (d0 + d1) + (d2 + d3);
+          s2 = fmaf(d0, d0, fmaf(d1, d1, fmaf(d2, d2, fmaf(d3, d3, s2))));
         }
         tmem_st_32x32b_x32(t_addr + c * 32, v);            // stash for pass 2
         __syncwarp();                                      // every lane has read this residual buffer
@@ -328,16 +344,20 @@ gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
         }
       }
       {
+        // this partial's (mean, centred sum of squares) over its 128 columns
+        constexpr float kInvPart = 1.0f / (NCHUNK * 32);
+        const float mean_p = fmaf(s1, kInvPart, piv);
+        const float m2_p = fmaxf(fmaf(-s1, s1 * kInvPart, s2), 0.f);
         const uint32_t off = ((slot * 6u + my_src) * 128u + static_cast<uint32_t>(row_in_cta)) * 8u;
         if (async_stats) {
           if (ew == 0 && lane == 0) mbar_arrive_expect_tx(&stats_bar[slot], 6u * 128u * 8u);   // what this CTA will receive
           const uint32_t bar_local = smem_u32(&stats_bar[slot]);
 #pragma unroll
           for (uint32_t pp = 0; pp < 3; ++pp)
-            st_async_f32x2(mapa_u32(stats_base + off, pp * 2 + half_m), s1, s2, mapa_u32(bar_local, pp * 2 + half_m));
+            st_async_f32x2(mapa_u32(stats_base + off, pp * 2 + half_m), mean_p, m2_p, mapa_u32(bar_local, pp * 2 + half_m));
         } else {
 #pragma unroll
-          for (uint32_t pp = 0; pp < 3; ++pp) st_cluster_f32x2(mapa_u32(stats_base + off, pp * 2 + half_m), s1, s2);
+          for (uint32_t pp = 0; pp < 3; ++pp) st_cluster_f32x2(mapa_u32(stats_base + off, pp * 2 + half_m), mean_p, m2_p);
           fence_acq_rel_cluster();
           __syncwarp();
           if (lane == 0) {
@@ -351,14 +371,22 @@ gemm_ln_f16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
       if (async_stats) mbar_wait(&stats_bar[slot], (it >> 1) & 1u);
       else mbar_wait_cluster(&stats_bar[slot], (it >> 1) & 1u);
       if (tr) stamp(it, 8);
-      float S1 = 0.f, S2 = 0.f;
+      float mean, var;
       {
+        // Chan et al.: mean = sum mean_p / 6, M2 = sum M2_p + 128 sum (mean_p - mean)^2.  The partial means are taken
+        // relative to partial 0 (differences of nearby values: exact), so the row mean is never rounded at 6 |mean|.
         const float2* st = reinterpret_cast<const float2*>(smem + Cfg::OFF_STATS) + (slot * 6) * 128 + row_in_cta;
+        const float m0 = st[0].x;
+        float dsum = 0.f, m2 = 0.f;
 #pragma unroll
-        for (int src = 0; src < 6; ++src) { const float2 p2 = st[src * 128]; S1 += p2.x; S2 += p2.y; }
+        for (int src = 0; src < 6; ++src) { const float2 p2 = st[src * 128]; dsum += p2.x - m0; m2 += p2.y; }
+        const float dm = dsum * (1.0f / 6.0f);
+        float between = 0.f;
+#pragma unroll
+        for (int src = 0; src < 6; ++src) { const float e = (st[src * 128].x - m0) - dm; between = fmaf(e, e, between); }
+        mean = m0 + dm;
+        var = fmaf(static_cast<float>(NCHUNK * 32), between, m2) * (1.0f / Cfg::N);
       }
-      const float mean = S1 * (1.0f / Cfg::N);
-      const float var = fmaxf(S2 * (1.0f / Cfg::N) - mean * mean, 0.f);
       const float rstd = 1.0f / sqrtf(var + eps);
       // ---------------- pass 2: normalise, stage, TMA-store fp32 + fp16 ----------------
       tmem_ld_32x32b_x32(t_addr, r[0]);
