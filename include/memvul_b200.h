@@ -76,9 +76,10 @@ typedef struct memvul_bert_weights {
 int memvul_abi_version(void);
 const char* memvul_last_error(void);
 
-/* Bytes of scratch memvul_encoder_forward needs for B sequences padded to S tokens with these flags.  With
- * MEMVUL_ENC_PACKED the workspace must be zero-initialised once before its first use (afterwards it only ever holds
- * finite values this library wrote), because rows past the last token of a partially filled tile are read. */
+/* Bytes of scratch memvul_encoder_forward needs for B sequences padded to S tokens with these flags.  The workspace
+ * needs no initialisation and may be reused for batches of any shape: every row a call reads is first written by that
+ * call (with MEMVUL_ENC_PACKED, the rows past the last token that partially filled tiles and the last sequence's key
+ * block read are zero-filled by the call's embedding kernel). */
 size_t memvul_encoder_workspace_bytes(const memvul_bert_weights* w, int B, int S, int flags);
 
 /* Replaces PretrainedTransformerEmbedder.forward / HF BertModel.forward

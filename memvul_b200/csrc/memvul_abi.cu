@@ -510,23 +510,27 @@ int layernorm_impl(const float* y, const float* g, const float* b, float eps, fl
   return MEMVUL_OK;
 }
 
+// qkv / ctx / ffn (nullable, packed layout only): the encoder's scratch matrices whose rows past the last token the
+// tail blocks zero-fill along with x32 / x16 (rowwise.cuh)
 int embed_impl(const memvul_bert_weights* w, const int64_t* ids, const int64_t* tids, const int32_t* lens,
-               const int32_t* row_start, int B, int S, float* x32, void* x16, int32_t* bad, cudaStream_t st) {
-  // 8 token rows per block, blocks never straddle sequences; packed layout: + 32 tail blocks that zero-fill the rows
-  // up to the next 256-row tile boundary
-  const int blocks = B * ((S + 7) / 8) + (row_start ? 32 : 0);
+               const int32_t* row_start, int B, int S, float* x32, void* x16, int32_t* bad, cudaStream_t st,
+               void* qkv = nullptr, void* ctx = nullptr, void* ffn = nullptr) {
+  // 8 token rows per block, blocks never straddle sequences; packed layout: + the tail blocks that zero-fill the rows
+  // past the last token
+  const int blocks = B * ((S + 7) / 8) + (row_start ? mv::kEmbedTailBlocks : 0);
   auto ll = [](const int64_t* p) { return reinterpret_cast<const long long*>(p); };
+  auto h = [](void* p) { return reinterpret_cast<__half*>(p); };
   LaunchScope ls(KC_EMBED_LN, st);
   if (w->hidden == 768)
     mv::embed_layernorm_kernel<6><<<blocks, 256, 0, st>>>(ll(ids), ll(tids), w->word_emb, w->pos_emb, w->type_emb,
-                                                          w->emb_ln_g, w->emb_ln_b, w->ln_eps, x32,
-                                                          reinterpret_cast<__half*>(x16), B, S, w->vocab, w->type_vocab,
-                                                          lens, row_start, bad);
+                                                          w->emb_ln_g, w->emb_ln_b, w->ln_eps, x32, h(x16), B, S,
+                                                          w->vocab, w->type_vocab, lens, row_start, bad, h(qkv), h(ctx),
+                                                          h(ffn), w->intermediate);
   else if (w->hidden == 128)
     mv::embed_layernorm_kernel<1><<<blocks, 256, 0, st>>>(ll(ids), ll(tids), w->word_emb, w->pos_emb, w->type_emb,
-                                                          w->emb_ln_g, w->emb_ln_b, w->ln_eps, x32,
-                                                          reinterpret_cast<__half*>(x16), B, S, w->vocab, w->type_vocab,
-                                                          lens, row_start, bad);
+                                                          w->emb_ln_g, w->emb_ln_b, w->ln_eps, x32, h(x16), B, S,
+                                                          w->vocab, w->type_vocab, lens, row_start, bad, h(qkv), h(ctx),
+                                                          h(ffn), w->intermediate);
   else
     return fail(MEMVUL_E_INVALID, "embedding supports hidden in {128, 768}, got %d", w->hidden);
   CUDA_TRY(cudaGetLastError());
@@ -824,7 +828,10 @@ int memvul_encoder_forward(const memvul_bert_weights* w, const int64_t* token_id
   const int* m_dev = packed ? row_start + B : nullptr;           // device-side row count T = sum(lens)
   // residual stream: the caller's hidden_out, except for a packed full-output run (unpacked at the end)
   float* x32 = (packed && !cls_only) ? ws.x32_packed : hidden_out;
-  if (int rc = embed_impl(w, token_ids, type_ids, lens, rs, B, S, x32, ws.x16, bad_flag, st)) return rc;
+  // packed: the embedding also zero-fills the scratch rows past the last token that tiles and key blocks read but no
+  // kernel of this call writes, so the workspace's previous contents never reach a result
+  if (int rc = embed_impl(w, token_ids, type_ids, lens, rs, B, S, x32, ws.x16, bad_flag, st, ws.qkv, ws.ctx, ws.ffn))
+    return rc;
   for (int l = 0; l < w->layers; ++l) {
     const memvul_bert_layer& L = w->layer[l];
     if (cls_only && l == w->layers - 1) {

@@ -102,31 +102,43 @@ __global__ void __launch_bounds__(256) unpack_rows_kernel(const float* __restric
 // (custom_PTM_embedder.py:199-202).  Out-of-range ids are clamped AND reported: bit 1 of *bad is set, which the host
 // turns into the error the reference raises (torch.embedding index error; custom_PTM_embedder.py:205 for type ids).
 // Padded layout (row_start == nullptr): output row b*S + s for every s < S.
-// Packed layout: only s < lens[b] is computed and lands at row row_start[b] + s; the rows between the last token and
-// the next 256-row GEMM tile boundary are zero-filled so that nothing non-finite can enter a partially filled tile.
+// Packed layout: only s < lens[b] is computed and lands at row row_start[b] + s.  The encoder's kernels also read rows
+// past the last token T that none of them writes: whole 256-row GEMM tiles, and the last sequence's ragged key block
+// (up to 63 rows past T, which P = 0 multiplies: a NaN there would still poison the sequence).  So the tail blocks
+// zero-fill rows [T, round_up(T, 256) + 64) (clipped to the B*S-row buffers) of x32, x16 and of the encoder's scratch
+// matrices qkv [*, 3H], ctx [*, H], ffn [*, inter] (each nullable), whatever the memory held before.
+constexpr int kEmbedTailBlocks = (256 + 64) / 8;
 template <int NV>
 __global__ void __launch_bounds__(256) embed_layernorm_kernel(
     const long long* __restrict__ ids, const long long* __restrict__ type_ids, const float* __restrict__ word,
     const float* __restrict__ pos, const float* __restrict__ type, const float* __restrict__ gamma,
     const float* __restrict__ beta, float eps, float* __restrict__ x32, __half* __restrict__ x16, int B, int S,
-    int vocab, int type_vocab, const int* __restrict__ lens, const int* __restrict__ row_start, int* __restrict__ bad) {
+    int vocab, int type_vocab, const int* __restrict__ lens, const int* __restrict__ row_start, int* __restrict__ bad,
+    __half* __restrict__ qkv, __half* __restrict__ ctx, __half* __restrict__ ffn, int inter) {
   constexpr int H = NV * 128;
   const int lane = threadIdx.x & 31;
   const int chunks = (S + 7) >> 3;                          // 8 rows (warps) per block, blocks never straddle sequences
   const int b = blockIdx.x / chunks;
   const int s = (blockIdx.x - b * chunks) * 8 + (threadIdx.x >> 5);
   if (b >= B) {
-    // packed layout only: tail blocks zero-fill rows [T, round_up(T, 256)) (clipped to the buffer)
+    // packed layout only: tail blocks, one row per warp
     const int T = row_start[B];
-    const int r = T + (blockIdx.x - B * chunks) * 8 + (threadIdx.x >> 5);
-    const int end = min(((T + 255) >> 8) << 8, B * S);
-    if (r < end) {
+    const size_t r = static_cast<size_t>(T + (blockIdx.x - B * chunks) * 8 + (threadIdx.x >> 5));
+    const int end = min((((T + 255) >> 8) << 8) + 64, B * S);
+    if (r < static_cast<size_t>(end)) {
 #pragma unroll
       for (int i = 0; i < NV; ++i) {
         const int col = i * 128 + lane * 4;
-        *reinterpret_cast<float4*>(x32 + static_cast<size_t>(r) * H + col) = make_float4(0.f, 0.f, 0.f, 0.f);
-        *reinterpret_cast<uint2*>(x16 + static_cast<size_t>(r) * H + col) = make_uint2(0u, 0u);
+        *reinterpret_cast<float4*>(x32 + r * H + col) = make_float4(0.f, 0.f, 0.f, 0.f);
+        *reinterpret_cast<uint2*>(x16 + r * H + col) = make_uint2(0u, 0u);
       }
+      auto zero_row = [&](__half* m, int cols) {           // 16-byte stores: cols is a multiple of 128
+        if (m)
+          for (int c = lane * 8; c < cols; c += 256) *reinterpret_cast<uint4*>(m + r * cols + c) = make_uint4(0u, 0u, 0u, 0u);
+      };
+      zero_row(qkv, 3 * H);
+      zero_row(ctx, H);
+      zero_row(ffn, inter);
     }
     return;
   }

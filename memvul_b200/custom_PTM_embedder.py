@@ -103,12 +103,11 @@ class PretrainedTransformerEmbedder(TokenEmbedder):
     def workspace(self, B: int, S: int, device: torch.device, flags: int = 0) -> torch.Tensor:
         need = self.packed().workspace_bytes(B, S, flags)
         if self._workspace is None or self._workspace.numel() < need or self._workspace.device != device:
-            # zero-initialised once (include/memvul_b200.h: the packed execution reads rows past the last token of a
-            # partially filled tile, which must be finite); grown geometrically so a stream of growing batches
-            # does not reallocate every step
+            # reused for every batch shape and never initialised (include/memvul_b200.h: each call writes every row it
+            # reads); grown geometrically so a stream of growing batches does not reallocate every step
             grow = 0 if self._workspace is None or self._workspace.device != device else self._workspace.numel() * 5 // 4
             self._workspace = None
-            self._workspace = torch.zeros(max(need, grow), dtype=torch.uint8, device=device)
+            self._workspace = torch.empty(max(need, grow), dtype=torch.uint8, device=device)
         return self._workspace
 
     def encode(self, token_ids: torch.Tensor, lens: torch.Tensor, type_ids: Optional[torch.Tensor] = None,

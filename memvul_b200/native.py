@@ -264,7 +264,7 @@ def encoder_forward(w: PackedBert, token_ids: torch.Tensor, lens: torch.Tensor,
     flags = encoder_flags(w, cls_only, row_start is not None)   # a PackedBert(precise=True) selects the accuracy mode
     need = w.workspace_bytes(B, S, flags)
     if workspace is None or workspace.numel() < need:
-        workspace = torch.zeros(need, dtype=torch.uint8, device=token_ids.device)   # zero-init: header contract (PACKED)
+        workspace = torch.empty(need, dtype=torch.uint8, device=token_ids.device)   # no initialisation needed (header)
     if out is None:
         out = torch.empty(B, S, w.hidden, dtype=torch.float32, device=token_ids.device)
     with _on(token_ids):
